@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W           # our CUDA path (one rank per GPU under torchrun)
     python bench.py --impl reference --gpus N ...           # the reference's own CPU path on the host cores
+    python bench.py ... --dump-outputs DIR                  # also save the last timed step's outputs as DIR/<name>.npy
 
 A bench "step" = one batched Env.step over all replicas of a rank (hashed random agent + step kernel).
 Workload (config.workload): BASELINE.json configs[1] — CIM toy.4p_ssdd_l0.0, 1024 parallel envs per GPU,
@@ -59,7 +60,7 @@ def parse():
     ap.add_argument("--vm-count", type=int, default=10000, help="vm_scheduling: VMs in the synthetic trace")
     ap.add_argument("--vm-query-agent", action="store_true", help="vm_scheduling e2e: the host agent makes the reference agent's snapshot "
                     "query every step (3.3 MB D2H) instead of reading the decision row's remaining-cores extension")
-    ap.add_argument("--vm-trace-dir", default="", help="vm_scheduling: where the synthetic trace is written (default: a temp dir)")
+    ap.add_argument("--vm-trace-dir", default="", help="vm_scheduling: where the synthetic trace is written and reused (default: a fresh temporary directory, removed at exit)")
     ap.add_argument("--max-snapshots", type=int, default=0, help="0 = keep every frame (reference default)")
     ap.add_argument("--no-flush", action="store_true", help="do not flush L2 between timed steps")
     ap.add_argument("--cpu-seconds", type=float, default=10.0, help="budget of the cpu_baseline leg")
@@ -73,7 +74,33 @@ def parse():
                     "1 k / 8 k / 64 k envs per GPU, short runs; the line's top-level keys are the first (headline) entry's")
     ap.add_argument("--matrix-sizes", default="1024,8192,65536")
     ap.add_argument("--skip-extras", action="store_true", help="cim: only the contract keys (value, e2e, roofline, cpu_baseline, clocks)")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write what the timed path returned in its last step (decision rows, metrics) to DIR/<name>.npy as float64; "
+                         "with --matrix, the headline entry's")
     return ap.parse_args()
+
+
+DUMP_LIMIT = 64 << 20  # bytes of all --dump-outputs files together
+
+
+def dump_outputs(out_dir, arrays, rank, world):
+    """--dump-outputs: one float64 .npy per array (integer outputs convert exactly), rows indexed by replica.  Past
+    DUMP_LIMIT a fixed, seeded sample of replica rows is kept, the same for every array, and its indices are written as
+    replica_rows.npy.  Ranks other than 0 add _rank<r> to the names."""
+    import numpy as np
+
+    arrays = {k: np.asarray(v, np.float64) for k, v in arrays.items()}
+    n = len(next(iter(arrays.values())))
+    row_bytes = sum(a[0].nbytes for a in arrays.values()) + 8
+    keep = min(n, (DUMP_LIMIT // world - 128 * (len(arrays) + 1)) // row_bytes)  # (128: .npy header)
+    if keep < n:
+        rows = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        arrays = {k: a[rows] for k, a in arrays.items()}
+        arrays["replica_rows"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    suffix = f"_rank{rank}" if rank else ""
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}{suffix}.npy"), a)
 
 
 # ----------------------------------------------------------------------------------------------- clocks
@@ -132,6 +159,14 @@ class ClockSampler:
 
 
 # ----------------------------------------------------------------------------------------------- reference arm
+def reference_built() -> bool:
+    """oracle/_ref holds the reference's compiled package (oracle/build_ref.sh also stages its Python sources on their own,
+    which cannot run the simulator)"""
+    import glob
+
+    return bool(glob.glob(os.path.join(ROOT, "oracle", "_ref", "maro", "backends", "frame*.so")))
+
+
 def run_reference(args, rank, world):
     """The reference's own CPU implementation on the host cores: maro.vector_env.VectorEnv(batch_num=cpu_count)
     from oracle/_ref (the unmodified reference built by oracle/build_ref.sh) when present, else the C port."""
@@ -149,7 +184,7 @@ def run_reference(args, rank, world):
         return run_reference_vm(args, line, ref_root, cores)
     if args.scenario == "citi_bike":
         return run_reference_bike(args, line, ref_root, cores)
-    if os.path.isdir(os.path.join(ref_root, "maro")):
+    if reference_built():
         os.environ["SKIP_DEPLOYMENT"] = "TRUE"
         os.environ.setdefault("DEFAULT_BACKEND_NAME", "dynamic")  # the Cython/C++ RawBackend the north-star names
         sys.path.insert(0, ref_root)
@@ -221,7 +256,7 @@ def run_reference_bike(args, line, ref_root, cores):
     ticks = min(args.ticks, 2880) if args.ticks != 1000 else 1440
     line["config"] = {"workload": f"citi_bike toy.3s_4t (frozen trace), {ticks} ticks, greedy top-1 agent, snapshot_resolution 10",
                       "replicas": cores}
-    if os.path.isdir(os.path.join(ref_root, "maro")):
+    if reference_built():
         os.environ["SKIP_DEPLOYMENT"] = "TRUE"
         sys.path.insert(0, ref_root)
         sys.path.insert(1, os.path.join(ref_root, "_stubs"))
@@ -284,7 +319,7 @@ def run_reference_vm(args, line, ref_root, cores):
     line["config"] = {"workload": f"vm_scheduling synthetic azure.2019.10k-scale trace ({args.vm_count} VMs, 100 PMs, {ticks} ticks), best-fit agent",
                       "replicas": cores}
     line["dtype"] = "int32+f64"
-    if os.path.isdir(os.path.join(ref_root, "maro")):
+    if reference_built():
         import yaml
 
         os.environ["SKIP_DEPLOYMENT"] = "TRUE"
@@ -380,7 +415,7 @@ def reference_inprocess(scenario, topology, ticks, seconds):
     import subprocess
 
     out = {}
-    if not os.path.isdir(os.path.join(ROOT, "oracle", "_ref", "maro")):
+    if not reference_built():
         return out
     for backend in ("static", "dynamic"):
         try:
@@ -423,22 +458,30 @@ def cpu_baseline_bike(args, topo):
                      "citi_bike", bike_toy_config_dir(), topo.max_tick)
 
 
+_HOST_AGENT = None
+
+
 def load_host_agent():
-    """Compile (gcc) and load tools/host_agent.c — the host-side agent of the e2e leg."""
+    """Compile (gcc) and load tools/host_agent.c — the host-side agent of the e2e leg.  The library is built in a
+    temporary directory, so that the benchmark writes nothing into the source tree (which may be read-only)."""
+    global _HOST_AGENT
+    if _HOST_AGENT is not None:
+        return _HOST_AGENT
     import ctypes
     import subprocess
+    import tempfile
 
     src = os.path.join(ROOT, "tools", "host_agent.c")
-    out = os.path.join(ROOT, "tools", "_build", "libhost_agent.so")
-    if not os.path.isfile(out) or os.path.getmtime(out) < os.path.getmtime(src):
-        os.makedirs(os.path.dirname(out), exist_ok=True)
+    with tempfile.TemporaryDirectory(prefix="maro_b200_bench_") as d:
+        out = os.path.join(d, "libhost_agent.so")
         subprocess.check_call(["gcc", "-O2", "-fopenmp", "-pthread", "-shared", "-fPIC", src, "-o", out])
-    lib = ctypes.CDLL(out)
+        lib = ctypes.CDLL(out)  # stays mapped after the directory is removed
     lib.agent_random.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_int, ctypes.c_uint32, ctypes.c_uint32]
     lib.agent_greedy.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_int, ctypes.c_int]
     lib.agent_best_fit.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_void_p,
                                    ctypes.c_void_p, ctypes.c_int, ctypes.c_int]
     lib.agent_best_fit_row.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_int, ctypes.c_int]
+    _HOST_AGENT = lib
     return lib
 
 
@@ -450,8 +493,13 @@ def vm_workload(args):
     import vm_trace_gen
 
     ticks = 8638 if args.ticks == 1000 else args.ticks
-    rank = os.environ.get("RANK", "0")  # one copy per rank: the ranks of a torchrun job generate it concurrently
-    d = args.vm_trace_dir or os.path.join(tempfile.gettempdir(), f"maro_b200_vm_trace_{args.vm_count}_{ticks}_r{rank}")
+    d = args.vm_trace_dir
+    if not d:  # a fresh directory per process (and so per rank), removed at exit
+        import atexit
+        import shutil
+
+        d = tempfile.mkdtemp(prefix="maro_b200_vm_trace_")
+        atexit.register(shutil.rmtree, d, True)
     vm_path, cpu_path = vm_trace_gen.generate(d, args.vm_count, ticks)
     return vm_trace_gen.azure_like_config(vm_path, cpu_path), ticks
 
@@ -607,13 +655,15 @@ def run_cim(args, rank, local_rank, world):
     """CIM arm.  `value`: resident rollouts — maro_cim_rollout_device fuses `chunk` env-steps per launch with the hashed
     hello-world agent as a device callback (replica blocks stay in shared memory; snapshot rows stream to the HBM ring).
     `e2e`: the host-buffer call maro_cim_step_pinned (resident session: command rows / decision rows through mapped
-    pinned memory) with the agent on the host.  Episode ends are detected from the DONE status column the device returns."""
+    pinned memory) with the agent on the host.  Episode ends come from the oracle's episode length and are checked against
+    the DONE status column the device returns."""
     import numpy as np
     import torch
     import torch.distributed as dist
 
     from maro_b200.batch import CimBatch
     from maro_b200.scenarios.cim.topology import build_topology, load_config
+    from oracle.cim_oracle import CimOracle  # episode length only
 
     torch.cuda.set_device(local_rank)
     if world > 1 and not dist.is_initialized():
@@ -638,48 +688,65 @@ def run_cim(args, rank, local_rank, world):
     def all_done():  # the `done` the reference's step returns: every replica answered DONE / FINISHED
         return bool((status != 0).all().item())
 
+    # An episode takes the same number of batched env-steps whatever the actions (one per decision event, plus the final
+    # one); with several seeds the longest counts, shorter replicas idle at DONE until the reset.
+    spe = max(CimOracle(t).run_episode(0)[0] for t in topos)
+    pos = {"i": 0}  # batched env-steps into the current episode
+
+    def next_episode():
+        """Env.reset once the episode is over (the first env-step of an episode ignores its action: generator start)"""
+        if pos["i"] < spe:
+            return 0
+        env.reset()
+        pos["i"] = 0
+        return 1
+
+    def check_done():
+        """the status column read back: every replica reports DONE exactly when the planned episode ends"""
+        assert all_done() == (pos["i"] == spe), f"episode end at env-step {pos['i']}, the oracle's episode has {spe}"
+
     # ------------------------------------------------------------------ value: fused resident rollouts
     def timed_rollouts(total_steps, chunk, timed):
-        """runs `total_steps` batched env-steps in launches of <= chunk; returns (device ms incl. resets, kernel ms, launches)"""
-        evs, launches, left, done = [], 0, total_steps, False
+        """exactly `total_steps` batched env-steps in launches of <= chunk that end at episode ends at the latest (the
+        kernel stops a launch at DONE); returns (device ms incl. resets, kernel ms, launches)"""
+        evs, launches, left = [], 0, total_steps
         while left > 0:
-            n = min(chunk, left)
             if flush is not None and timed:
                 flush.fill_(1)
             e = [torch.cuda.Event(enable_timing=True) for _ in range(3)]
             e[0].record(stream)
-            if done:
-                env.reset()
-                launches += 1
+            launches += next_episode()
+            n = min(chunk, left, spe - pos["i"])
             e[1].record(stream)
             env.rollout_device(dec.data_ptr(), met.data_ptr(), n, 1, 0, base)
             e[2].record(stream)
             launches += 1
             evs.append(e)
             left -= n
-            done = all_done()
+            pos["i"] += n
+            check_done()
         torch.cuda.synchronize()
-        return (sum(e[0].elapsed_time(e[2]) for e in evs), sum(e[1].elapsed_time(e[2]) for e in evs), launches, done)
+        return sum(e[0].elapsed_time(e[2]) for e in evs), sum(e[1].elapsed_time(e[2]) for e in evs), launches
 
     def timed_launch_per_step(total_steps, timed):
-        evs, launches, done = [], 0, False
+        evs, launches = [], 0
         for k in range(total_steps):
             if flush is not None and timed:
                 flush.fill_(1)
             e = [torch.cuda.Event(enable_timing=True) for _ in range(3)]
             e[0].record(stream)
-            if done:
-                env.reset()
-                launches += 1
+            launches += next_episode()
             env.random_policy_device(dec.data_ptr(), act.data_ptr(), 0, base)
             e[1].record(stream)
             env.step_device(dec.data_ptr(), met.data_ptr(), act.data_ptr())
             e[2].record(stream)
             launches += 2
             evs.append(e)
-            done = (k % 16 == 15) and all_done()  # the status column is read back every 16 steps
+            pos["i"] += 1
+            if k % 16 == 15 or pos["i"] == spe:  # (read back every 16 steps and at each episode end)
+                check_done()
         torch.cuda.synchronize()
-        return (sum(e[0].elapsed_time(e[2]) for e in evs), sum(e[1].elapsed_time(e[2]) for e in evs), launches, done)
+        return sum(e[0].elapsed_time(e[2]) for e in evs), sum(e[1].elapsed_time(e[2]) for e in evs), launches
 
     chunk = max(1, min(args.chunk, args.steps))
     warm = max(args.warmup, 3)
@@ -692,22 +759,25 @@ def run_cim(args, rank, local_rank, world):
     torch.cuda.synchronize()
     sampler.start()
     wall0 = time.perf_counter()
-    total_ms, kernel_ms, launches, _ = primary(args.steps, True)
+    total_ms, kernel_ms, launches = primary(args.steps, True)
     wall = time.perf_counter() - wall0
     clocks = sampler.stop()
     if world > 1:
         dist.barrier()
     c1 = env.counters().sum(0)
     d_steps, d_ticks, d_events, d_snaps = (int(x) for x in (c1 - c0))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"decisions": dec.cpu(), "metrics": met.cpu()}, rank, world)
 
     extras = {}
     if not args.skip_extras and not args.launch_per_step:  # the one-launch-per-Env.step path, for comparison
         env.reset()
         dec.zero_()
+        pos["i"] = 0
         n = min(args.steps, 500)
         timed_launch_per_step(warm, False)
         k0 = env.counters().sum(0)
-        ms, kms, _, _ = timed_launch_per_step(n, True)
+        ms, kms, _ = timed_launch_per_step(n, True)
         k1 = env.counters().sum(0)
         extras["launch_per_step"] = {"value": float(k1[0] - k0[0]) / (ms / 1000.0), "unit": "env-steps/s", "steps": n,
                                      "us_per_step": 1000.0 * ms / n, "kernel_us": 1000.0 * kms / n,
@@ -945,25 +1015,27 @@ def run_ours(args, rank, local_rank, world):
     launches = 2 * args.steps
 
     def timed_rollouts(total_steps, chunk, timed):
-        """`total_steps` batched env-steps in launches of <= chunk (greedy agent as a device callback); Env.reset when every
-        replica reports DONE.  Returns (device ms incl. resets, kernel ms, launches)."""
-        evs, n_launch, left, done = [], 0, total_steps, False
+        """exactly `total_steps` batched env-steps in launches of <= chunk (the rule-based agent as a device callback) that
+        end at episode ends at the latest (the kernel stops a launch at DONE); Env.reset at each episode end.  Returns (device ms incl. resets, kernel ms, launches)."""
+        evs, n_launch, left = [], 0, total_steps
         while left > 0:
-            n = min(chunk, left)
             if flush is not None and timed:
                 flush.fill_(1)
             e = [torch.cuda.Event(enable_timing=True) for _ in range(3)]
             e[0].record(stream)
-            if done:
+            if pos["i"] > 0 and pos["i"] % steps_per_episode == 0:
                 env.reset()
                 n_launch += 1
+            n = min(chunk, left, steps_per_episode - pos["i"] % steps_per_episode)
             e[1].record(stream)
             env.rollout_device(dec.data_ptr(), met.data_ptr(), n)
             e[2].record(stream)
             n_launch += 1
             evs.append(e)
             left -= n
-            done = bool((dec[:, 6] != 0).all().item())
+            pos["i"] += n
+            done = bool((dec[:, 6] != 0).all().item())  # every replica reports DONE exactly when the planned episode ends
+            assert done == (pos["i"] % steps_per_episode == 0), f"episode end at env-step {pos['i']}, the oracle's has {steps_per_episode}"
         torch.cuda.synchronize()
         return sum(e[0].elapsed_time(e[2]) for e in evs), sum(e[1].elapsed_time(e[2]) for e in evs), n_launch
 
@@ -997,6 +1069,14 @@ def run_ours(args, rank, local_rank, world):
         kernel_ms = sum(e[1].elapsed_time(e[2]) for e in events)
     c1 = env.counters().sum(0)
     d_steps, d_ticks, d_events, d_snaps = (int(x) for x in (c1 - c0))
+    if args.dump_outputs:
+        m = met.cpu().numpy()
+        if vm:  # these slots hold float64 bit patterns: decode them as the metrics dict does (_abi.vm_metrics)
+            from maro_b200._abi import VM_METRIC_FLOAT
+
+            m = m.astype(np.float64)
+            m[:, VM_METRIC_FLOAT] = met.cpu().numpy()[:, VM_METRIC_FLOAT].view(np.float64)
+        dump_outputs(args.dump_outputs, {"decisions": dec.cpu(), "metrics": m}, rank, world)
     if fused:  # the extra legs below drive the per-step path from a fresh episode
         env.reset()
         dec.zero_()
@@ -1233,8 +1313,8 @@ def main():
                 a = copy.copy(args)
                 a.scenario, a.replicas, a.skip_extras, a.graph_chunk = scenario, B, True, 0
                 a.topology, a.ticks = "toy.4p_ssdd_l0.0", 1000
-                a.steps = args.steps if B <= 8192 else max(64, args.steps // 4)
                 a.cpu_seconds = min(args.cpu_seconds, 3.0) if B == sizes[0] else 0.0
+                a.dump_outputs = args.dump_outputs if (scenario, B) == ("cim", sizes[0]) else ""
                 try:
                     ln = run(a)
                 except Exception as ex:  # one configuration failing (e.g. out of memory) must not lose the others

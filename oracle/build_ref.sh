@@ -12,6 +12,7 @@
 set -euo pipefail
 HERE="$(cd "$(dirname "${BASH_SOURCE[0]}")" && pwd)"
 REF="${MARO_REFERENCE_ROOT:-/root/reference}"
+PY="${PYTHON:-python}"  # the interpreter whose Cython / setuptools build the package
 OUT="$HERE/_ref"
 if [ ! -d "$REF/maro" ]; then
   echo "build_ref: $REF not present (GPU box) - keeping prebuilt $OUT" >&2
@@ -51,19 +52,38 @@ copy_examples() {
   [ -f "$REF/examples/__init__.py" ] && cp "$REF/examples/__init__.py" "$OUT/examples/" || true
   [ -f "$REF/examples/cim/__init__.py" ] && cp "$REF/examples/cim/__init__.py" "$OUT/examples/cim/" || true
 }
+# the package = python modules + built extension modules (if any) + topology/meta data files of $1/maro, into $OUT/maro
+copy_package() {
+  "$PY" - "$1" "$OUT" <<'PY'
+import os, shutil, sys
+src, dst = sys.argv[1], sys.argv[2]
+keep = (".py", ".so", ".yml", ".yaml", ".json", ".csv", ".txt", ".toml", ".bin")
+for root, _, files in os.walk(os.path.join(src, "maro")):
+    for f in files:
+        if f.endswith(keep):
+            rel = os.path.relpath(os.path.join(root, f), src)
+            os.makedirs(os.path.dirname(os.path.join(dst, rel)), exist_ok=True)
+            shutil.copy2(os.path.join(root, f), os.path.join(dst, rel))
+PY
+}
+# the example scripts first: the hello cases of tests/test_gpu_shim.py need only them, not the compiled package below
+copy_examples
+write_rl_stubs
 if [ -f "$OUT/maro/backends/frame.cpython-312-x86_64-linux-gnu.so" ] && [ -z "${FORCE:-}" ]; then
-  copy_examples
-  write_rl_stubs
   echo "build_ref: $OUT already built"; exit 0
 fi
+# then the Python sources on their own: maro.rl is pure Python and runs on the maro_b200 shim (the maro.rl cases of
+# tests/test_gpu_shim.py) even where the Cython build below fails; the compiled package replaces them
+rm -rf "$OUT/maro"
+copy_package "$REF"
 TMP="$(mktemp -d /tmp/maro_ref_build.XXXXXX)"
 trap 'rm -rf "$TMP"' EXIT
 cp -r "$REF/maro" "$REF/setup.py" "$REF/scripts" "$TMP/"
 [ -f "$REF/README.md" ] && cp "$REF/README.md" "$TMP/" || true
 cd "$TMP"
 export SKIP_DEPLOYMENT=TRUE
-python scripts/code_gen.py
-python - <<'PY'
+"$PY" scripts/code_gen.py
+"$PY" - <<'PY'
 import re, io
 p = "maro/backends/frame.pyx"
 s = open(p).read()
@@ -78,22 +98,11 @@ s = s.replace('format="f"', 'format="d"')
 open(p, "w").write(s)
 print("raw_backend.pyx: patched", n, "buffer formats")
 PY
-cython maro/backends/backend.pyx maro/backends/np_backend.pyx maro/backends/raw_backend.pyx maro/backends/frame.pyx \
+"$PY" -m cython maro/backends/backend.pyx maro/backends/np_backend.pyx maro/backends/raw_backend.pyx maro/backends/frame.pyx \
   --cplus -3 -E NODES_MEMORY_LAYOUT=ONE_BLOCK -X embedsignature=True
-python setup.py -q build_ext -i -j 8 2>&1 | tail -5
-rm -rf "$OUT"; mkdir -p "$OUT"
-# the installed package = python modules + built extension modules + topology/meta data files
-python - "$TMP" "$OUT" <<'PY'
-import os, shutil, sys
-src, dst = sys.argv[1], sys.argv[2]
-keep = (".py", ".so", ".yml", ".yaml", ".json", ".csv", ".txt", ".toml", ".bin")
-for root, _, files in os.walk(os.path.join(src, "maro")):
-    for f in files:
-        if f.endswith(keep):
-            rel = os.path.relpath(os.path.join(root, f), src)
-            os.makedirs(os.path.dirname(os.path.join(dst, rel)), exist_ok=True)
-            shutil.copy2(os.path.join(root, f), os.path.join(dst, rel))
-PY
+"$PY" setup.py -q build_ext -i -j 8 2>&1 | tail -5
+rm -rf "$OUT/maro"
+copy_package "$TMP"
 # import-time stubs for packages absent from this image (only touched by the citi_bike import chain)
 mkdir -p "$OUT/_stubs/holidays" "$OUT/_stubs/geopy"
 cat > "$OUT/_stubs/holidays/__init__.py" <<'PY'
@@ -115,6 +124,4 @@ def distance(a, b):
     h = math.sin((p2 - p1) / 2) ** 2 + math.cos(p1) * math.cos(p2) * math.sin(math.radians(lo2 - lo1) / 2) ** 2
     return _D(2 * 6371.0088 * math.asin(math.sqrt(h)))
 PY
-copy_examples
-write_rl_stubs
 echo "build_ref: built into $OUT"

@@ -130,13 +130,21 @@ def test_vm_float_queries_are_lifted_to_the_reference_float64_values():
 
 
 def test_reference_examples_run_unchanged_on_the_shim_emulated():
-    """maro import shim: hello_world/cim/hello.py, vector_env/hello.py and the maro.rl CIM sampler + DQN train step, unmodified"""
+    """maro import shim: hello_world/cim/hello.py and vector_env/hello.py, unmodified"""
     import test_gpu_shim as shim_cases
 
-    if not shim_cases.HAVE_REF:
-        pytest.skip("oracle/_ref/examples not built")
+    if not shim_cases.HAVE_EXAMPLES:
+        pytest.skip("oracle/_ref/examples not staged (oracle/build_ref.sh)")
     shim_cases.test_hello_world_cim_unchanged(emulate=True)
     shim_cases.test_vector_env_hello_unchanged(emulate=True)
+
+
+def test_rl_toolkit_runs_unchanged_on_the_shim_emulated():
+    """maro import shim: the maro.rl CIM sampler + DQN train step of examples/cim/rl, unmodified"""
+    import test_gpu_shim as shim_cases
+
+    if not (shim_cases.HAVE_RL and shim_cases.HAVE_EXAMPLES):
+        pytest.skip("oracle/_ref (maro.rl + examples) not staged (oracle/build_ref.sh)")
     shim_cases.test_rl_toolkit_sampler_and_train_step_unchanged(emulate=True)
 
 

@@ -204,7 +204,7 @@ def test_vm_vector_env_two_envs_and_pinned_api(pinned=True):
         assert decisions[0, 1] == int(gold["steps"][1][1]) and mets.shape == (2, 16)
 
 
-def test_vm_cuda_full_size_episode_matches_oracle():
+def test_vm_cuda_full_size_episode_matches_oracle(tmp_path):
     """BASELINE config #5 size: 2 048 replicas, 10 000 VMs, 100 PMs, 8 638 ticks (synthetic azure.2019.10k-scale trace,
     tools/vm_trace_gen.py), best-fit agent kernel, the whole episode device-resident.  All replicas must agree, the
     request bookkeeping must balance, and the final metrics / frame / counters must equal the oracle's."""
@@ -220,7 +220,7 @@ def test_vm_cuda_full_size_episode_matches_oracle():
     from oracle.vm_oracle import VmOracle
 
     ticks = 8638
-    vm_path, cpu_path = vm_trace_gen.generate(os.path.join(tempfile.gettempdir(), "maro_b200_vm_trace_test"), 10000, ticks)
+    vm_path, cpu_path = vm_trace_gen.generate(str(tmp_path), 10000, ticks)
     topo = build_vm_topology(vm_trace_gen.azure_like_config(vm_path, cpu_path), 0, ticks)
     assert topo.n_vm == 10000 and topo.n_pm == 100 and topo.error is None
     o = VmOracle(topo, 1, 8)
